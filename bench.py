@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W
     python bench.py --config c1|c2|c3|c4r|c4m|c5 ...         (the other BASELINE configs; lines kept under profiles/)
+    python bench.py ... --dump-outputs DIR                   (also writes the last timed step's output as DIR/*.npy)
 
 A "step" is one pass of the hot path (K1 ingest -> stable sort -> layout scan -> K4 place) over one batch of
 synthetic FASTQ chunks.  Workload (SURVEY.md 8d):
@@ -47,6 +48,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True       # the tree may be read-only; the benchmark leaves nothing in it
 
 METRIC = "reads_per_sec_binned"
 UNIT = "reads/s"
@@ -289,6 +291,67 @@ def block_dict(blk):
             "raw_head_size": blk.raw_head_size, "n_records": blk.n_records, "read_signature": blk.read_signature, "read_info": blk.read_info}
 
 
+DUMP_STREAMS = ("meta", "dna", "qua", "head")
+DUMP_STREAM_SAMPLE = 2 << 20          # bytes per stream (float32: 8 MB each)
+DUMP_BIN_SAMPLE = 1 << 17             # descriptor rows (9 float64 columns: 9 MB)
+DUMP_SEED = 20260
+
+
+def dump_outputs(out_dir, blocks):
+    """Writes the blocks of the last timed step as out_dir/<name>.npy, for comparing two builds output for output:
+
+      sizes.npy          float64 [chunk, 8]     n_records, n_bins, meta/dna/qua/head stream sizes, raw_dna_size, raw_head_size
+      sha256.npy         float64 [chunk, 5, 8]  SHA-256 of the meta, dna, qua, head streams and the bin descriptors, as 32-bit words
+      <stream>.npy       float32 [<= 2 Mi]      a seeded sample of the bytes of that stream, all chunks end to end
+      bins.npy           float64 [<= 128 Ki, 9] a seeded sample of descriptor rows: chunk, then the 8 fields of fsb_bin_desc
+
+    The whole output is gigabytes, so the values are sampled (42 MB in all) and the digests cover every byte.  The sample
+    positions depend only on the sizes, so two builds that agree on the sizes are sampled at the same positions."""
+    import hashlib
+    from concurrent.futures import ThreadPoolExecutor
+    from fastore_b200 import _native as N
+
+    def view(ptr, nbytes, dtype=np.uint8):
+        if not ptr or nbytes == 0:
+            return np.zeros(0, dtype=dtype)
+        return np.frombuffer((C.c_uint8 * int(nbytes)).from_address(ptr), dtype=dtype)
+
+    streams = [{s: view(getattr(b, s), getattr(b, s + "_size")) for s in DUMP_STREAMS} for b in blocks]
+    bins = [view(b.bins, int(b.n_bins) * N.BIN_DESC_DTYPE.itemsize, N.BIN_DESC_DTYPE) for b in blocks]
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    sizes = [[b.n_records, b.n_bins, b.meta_size, b.dna_size, b.qua_size, b.head_size, b.raw_dna_size, b.raw_head_size] for b in blocks]
+    np.save(out / "sizes.npy", np.array(sizes, dtype=np.float64).reshape(len(blocks), 8))
+    parts = [st[s] for st in streams for s in DUMP_STREAMS] + [np.frombuffer(bn.tobytes(), np.uint8) for bn in bins]
+    with ThreadPoolExecutor(max_workers=8) as ex:
+        digests = list(ex.map(lambda a: np.frombuffer(hashlib.sha256(a).digest(), ">u4"), parts))
+    sha = np.array(digests, dtype=np.float64).reshape(5, len(blocks), 8).transpose(1, 0, 2)
+    np.save(out / "sha256.npy", np.ascontiguousarray(sha))
+    rng = np.random.default_rng(DUMP_SEED)
+
+    def sample(arrays, k):
+        """Sorted seeded positions in the arrays laid end to end: (array index, position in it)."""
+        ends = np.cumsum([a.shape[0] for a in arrays], dtype=np.int64)
+        total = int(ends[-1]) if len(ends) else 0
+        pos = np.sort(rng.integers(0, total, min(k, total), dtype=np.int64)) if total else np.zeros(0, np.int64)
+        which = np.searchsorted(ends, pos, side="right")
+        return which, pos - np.concatenate(([0], ends[:-1]))[which]
+
+    for s in DUMP_STREAMS:
+        arrays = [st[s] for st in streams]
+        which, pos = sample(arrays, DUMP_STREAM_SAMPLE)
+        vals = np.concatenate([arrays[i][pos[which == i]] for i in range(len(arrays))]) if len(pos) else np.zeros(0, np.uint8)
+        np.save(out / f"{s}.npy", vals.astype(np.float32))
+    which, pos = sample(bins, DUMP_BIN_SAMPLE)
+    rows = np.zeros((len(pos), 9), dtype=np.float64)
+    rows[:, 0] = which
+    for i in range(len(bins)):
+        sel = which == i
+        for j, f in enumerate(N.BIN_DESC_DTYPE.names):
+            rows[sel, 1 + j] = bins[i][f][pos[sel]]
+    np.save(out / "bins.npy", rows)
+
+
 # -------------------------------------------------------------------------------------------------
 def run_b200_arm(args, w, name):
     import torch
@@ -434,6 +497,8 @@ def run_b200_arm(args, w, name):
     checked_records = int(sharding.sum_over_ranks(float(sum(int(chunks[ci].n_records) for ci in pick)), device="cuda"))
     if not ok:
         log(f"[rank {rank}] PARITY FAILURE: {detail}")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, raw_blocks)
     del raw_blocks, holder
 
     # ---- end to end through the C ABI with host buffers -----------------------------------------------
@@ -565,7 +630,11 @@ def main():
                     help="sub-batches fsb_run overlaps on two streams in the timed resident steps (FSB_OPT_RUN_SPLIT; 1 = one pass on one stream)")
     ap.add_argument("--parity-chunks", type=int, default=1, help="whole chunks per rank compared with the compiled reference (1 or 2)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0's chunks) to DIR/*.npy: sizes, digests and a seeded sample")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     name = args.config
     if name == "auto":

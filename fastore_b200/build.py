@@ -83,12 +83,13 @@ def build_cli(force=False, verbose=False) -> Path:
 
 def build_oracle(verbose=False) -> None:
     """Build the CPU checkers (test infrastructure): the C port always, the compiled reference only
-    when /root/reference exists (this container; the GPU box uses the prebuilt oracle/_ref)."""
+    when FASTORE_REFERENCE names a checkout of the reference's sources (into oracle/_ref)."""
     _run(["make", "-C", ROOT / "oracle", "port"], verbose)
-    if Path(os.environ.get("FASTORE_REFERENCE", "/root/reference")).is_dir():
-        _run(["make", "-C", ROOT / "oracle", "-j8", "ref"], verbose)
+    ref = os.environ.get("FASTORE_REFERENCE")
+    if ref and Path(ref).is_dir():
+        _run(["make", "-C", ROOT / "oracle", "-j8", f"REF={ref}", "ref"], verbose)
         if CUDA_LIB.exists():                      # the reference's fastore_bin with the C ABI bound in (integration/)
-            _run(["make", "-C", ROOT / "oracle", "ref_gpu"], verbose)
+            _run(["make", "-C", ROOT / "oracle", f"REF={ref}", "ref_gpu"], verbose)
 
 
 def build_all(force=False, verbose=False) -> None:

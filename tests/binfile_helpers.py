@@ -4,6 +4,8 @@ chain from Python (the block producer is the oracle in the CPU tier, the CLI use
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import json
 import subprocess
 from pathlib import Path
 
@@ -16,6 +18,7 @@ from fastore_b200 import synth
 ROOT = Path(__file__).resolve().parent.parent
 REF_DIR = ROOT / "oracle" / "_ref"
 CLI = ROOT / "fastore_b200" / "fastore_bin_b200"
+GOLDEN_FILES = ROOT / "tests" / "golden" / "bin_files.json"
 
 # never-initialised bytes of the 88-byte BinModuleConfig dump in the footer (SURVEY.md 8c): struct padding,
 # qvzOpts.uncompressed and the two char* of qv_options_t
@@ -151,6 +154,33 @@ def assert_bin_files_equal(a: Path, b: Path, headers: bool):
     if x != y:
         i = next(k for k in range(len(x)) if x[k] != y[k])
         raise AssertionError(f".bmeta differs at byte {i} (footer starts at {foot}, params end at {foot + 88}): {x[i]} vs {y[i]}")
+
+
+def bin_file_digests(prefix: Path, headers: bool) -> dict:
+    """SHA-256 of each bin file, the .bmeta with the never-initialised parameter bytes of its footer zeroed."""
+    out = {ext: hashlib.sha256(Path(str(prefix) + ext).read_bytes()).hexdigest() for ext in (".bdna", ".bqua") + ((".bhead",) if headers else ())}
+    x = bytearray(Path(str(prefix) + ".bmeta").read_bytes())
+    foot = int.from_bytes(x[0:8], "little")
+    for i in PARAM_MASK:
+        x[foot + i] = 0
+    out[".bmeta"] = hashlib.sha256(x).hexdigest()
+    return out
+
+
+def assert_reference_files(ours: Path, files, flags: dict, key: str, tmp: Path):
+    """Our bin files against what the reference's `fastore_bin e -t1` writes for the same input files: the reference itself
+    where oracle/_ref is built, its stored digests (tests/golden/bin_files.json, key `key`) elsewhere."""
+    headers = flags.get("headers", True)
+    if have_ref_tools():
+        run_reference_bin(files, tmp / "ref", flags)
+        assert_bin_files_equal(ours, tmp / "ref", headers)
+        return
+    want = json.loads(GOLDEN_FILES.read_text())[key]
+    assert [hashlib.sha256(Path(f).read_bytes()).hexdigest() for f in files] == want["input_sha256"], \
+        f"{key}: the synthetic generator wrote other input files than the golden digests were taken from"
+    got = bin_file_digests(ours, headers)
+    for ext, digest in want["files"].items():
+        assert got[ext] == digest, f"{key}: {ext} differs from the reference's file"
 
 
 def decode_with_reference(prefix: Path, out_files, paired: bool):

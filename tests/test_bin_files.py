@@ -6,7 +6,7 @@ import pytest
 
 import binfile_helpers as BF
 
-pytestmark = pytest.mark.skipif(not BF.have_ref_tools(), reason="oracle/_ref tools not built (no /root/reference here)")
+needs_ref_tools = pytest.mark.skipif(not BF.have_ref_tools(), reason="the reference's decoder and downstream tools (oracle/_ref) are not built")
 
 CASES = [
     ("se100_multichunk", dict(n=30000, L=100, paired=False, seed=201), dict(b=2)),
@@ -20,10 +20,9 @@ CASES = [
 @pytest.mark.parametrize("name,gen,flags", CASES, ids=[c[0] for c in CASES])
 def test_host_chain_reproduces_reference_files(tmp_path, name, gen, flags):
     files = BF.write_fastq(tmp_path, name, gen["n"], gen["L"], gen["paired"], gen["seed"], **{k: v for k, v in gen.items() if k not in ("n", "L", "paired", "seed")})
-    BF.run_reference_bin(files, tmp_path / "ref", flags)
     sizes = BF.host_chain(files, tmp_path / "ours", flags, BF.oracle_producer)
     assert len(sizes) >= (2 if "multichunk" in name else 1)
-    BF.assert_bin_files_equal(tmp_path / "ours", tmp_path / "ref", flags.get("headers", True))
+    BF.assert_reference_files(tmp_path / "ours", files, flags, name, tmp_path)
 
 
 @pytest.mark.gpu
@@ -31,9 +30,8 @@ def test_host_chain_reproduces_reference_files(tmp_path, name, gen, flags):
 def test_cli_reproduces_reference_files(tmp_path, name, gen, flags):
     assert BF.CLI.exists(), "fastore_bin_b200 is not built"
     files = BF.write_fastq(tmp_path, name, gen["n"], gen["L"], gen["paired"], gen["seed"], **{k: v for k, v in gen.items() if k not in ("n", "L", "paired", "seed")})
-    BF.run_reference_bin(files, tmp_path / "ref", flags)
     BF.run_cli(files, tmp_path / "ours", flags)
-    BF.assert_bin_files_equal(tmp_path / "ours", tmp_path / "ref", flags.get("headers", True))
+    BF.assert_reference_files(tmp_path / "ours", files, flags, name, tmp_path)
 
 
 @pytest.mark.gpu
@@ -42,11 +40,11 @@ def test_cli_with_device_side_parse_reproduces_reference_files(tmp_path, name, g
     """-D: the chunks go to the library as text alone and are parsed on the GPU (parse.cuh); the tables come back for the title
     statistics.  Same files as `fastore_bin e -t1`, CRLF and -C included."""
     files = BF.write_fastq(tmp_path, name, gen["n"], gen["L"], gen["paired"], gen["seed"], **{k: v for k, v in gen.items() if k not in ("n", "L", "paired", "seed")})
-    BF.run_reference_bin(files, tmp_path / "ref", flags)
     BF.run_cli(files, tmp_path / "ours", flags, device_parse=True, per_call=3)
-    BF.assert_bin_files_equal(tmp_path / "ours", tmp_path / "ref", flags.get("headers", True))
+    BF.assert_reference_files(tmp_path / "ours", files, flags, name, tmp_path)
 
 
+@needs_ref_tools
 @pytest.mark.gpu
 @pytest.mark.parametrize("paired", [False, True])
 def test_reference_decoder_reads_our_files(tmp_path, paired):
@@ -71,15 +69,15 @@ def test_cli_with_many_workers_is_byte_identical(tmp_path, workers, per_call):
     assert G >= 1
     files = BF.write_fastq(tmp_path, "mg", 60000, 150, True, 220)
     flags = dict(paired=True, b=2)
-    BF.run_reference_bin(files, tmp_path / "ref", flags)
     BF.run_cli(files, tmp_path / "ours", flags, gpus=G, workers=workers, per_call=per_call)
-    BF.assert_bin_files_equal(tmp_path / "ours", tmp_path / "ref", True)
+    BF.assert_reference_files(tmp_path / "ours", files, flags, "many_workers", tmp_path)
 
 
 DOWNSTREAM = [("se_c0_pack", False, False, dict(s=10, b=2)), ("pe_c1_rebin_pack", True, True, dict(paired=True, b=2)),
               ("se_c1_rebin_pack", False, True, dict(b=2))]
 
 
+@needs_ref_tools
 @pytest.mark.parametrize("name,paired,rebin,flags", DOWNSTREAM, ids=[d[0] for d in DOWNSTREAM])
 def test_reference_rebin_and_pack_consume_host_chain_files(tmp_path, name, paired, rebin, flags):
     """Mode C, downstream tools: fastore_rebin e -p2 -> fastore_pack e -> fastore_pack d (the reference's own pipeline,
@@ -92,6 +90,7 @@ def test_reference_rebin_and_pack_consume_host_chain_files(tmp_path, name, paire
         assert sorted(BF.fastq_records(src)) == sorted(BF.fastq_records(dec))
 
 
+@needs_ref_tools
 @pytest.mark.gpu
 @pytest.mark.parametrize("name,paired,rebin,flags", DOWNSTREAM, ids=[d[0] for d in DOWNSTREAM])
 def test_reference_rebin_and_pack_consume_cli_files(tmp_path, name, paired, rebin, flags):

@@ -108,15 +108,13 @@ def test_memchr_line_scanner_follows_skipline():
     assert _parse(bad, 1)[0] == N.FSB_ERR_INPUT and _parse(bad, 0)[0] == N.FSB_OK
 
 
-@pytest.mark.skipif(not BF.have_ref_tools(), reason="oracle/_ref tools not built (no /root/reference here)")
 def test_title_statistics_merged_per_chunk_equal_the_reference(tmp_path):
     """The CLI's parser threads gather the header-field statistics per chunk (fsh_titles) and the writer merges them in chunk
     order; the footer must be the one the reference writes from its record-by-record statistics."""
     files = BF.write_fastq(tmp_path, "in", 16000, 100, True, 250, header_comments=True)
     flags = dict(paired=True, b=2)
-    BF.run_reference_bin(files, tmp_path / "ref", flags)
     BF.host_chain(files, tmp_path / "ours", flags, BF.oracle_producer, merge_titles=True)
-    BF.assert_bin_files_equal(tmp_path / "ours", tmp_path / "ref", True)
+    BF.assert_reference_files(tmp_path / "ours", files, flags, "title_statistics", tmp_path)
 
 
 def test_large_requests_read_as_slices_reassemble_the_file(tmp_path):
