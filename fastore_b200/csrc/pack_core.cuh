@@ -169,12 +169,14 @@ template <int Q>
 FSB_HD uint32_t quality4(uint32_t b, uint32_t off4 /* offset * 0x01010101 */, uint32_t thr4 /* threshold * 0x01010101 */)
 {
     if (Q == 6) return gather4x6((b | 0x80808080u) - off4);             // (q - offset) & 63: the borrow guard bit 7 is masked off
-    const uint32_t d = ((b | 0x80808080u) - off4) ^ 0x80808080u;        // per byte (q - offset) mod 256, no borrow between bytes
     if (Q == 1)
-    {   // c >= binaryThreshold on the unsigned difference: a "negative" difference is large
-        const uint32_t ge = ((((d | 0x80808080u) - thr4) | d) >> 7) & 0x01010101u;
+    {   // c >= binaryThreshold on the unsigned difference: a "negative" difference is large.  The 1-bit mode takes every byte
+        // from the offset up, so c needs all eight bits: per byte (q - offset) mod 256, no borrow between bytes
+        const uint32_t c = ((b | 0x80808080u) - (off4 & 0x7F7F7F7Fu)) ^ ((b ^ ~off4) & 0x80808080u);
+        const uint32_t ge = ((((c | 0x80808080u) - thr4) | c) >> 7) & 0x01010101u;
         return gather4x1(ge);
     }
+    const uint32_t d = ((b | 0x80808080u) - off4) ^ 0x80808080u;        // per byte (q - offset) mod 256 for q < 128 (the table reads its low six bits)
     // quaToIdx_8bin (FastqPacker.cpp:41-64) of c & 63: [0,1]->0 [2,9]->1 [10,19]->2 [20,24]->3 [25,29]->4 [30,34]->5 [35,39]->6 >=40->7
     const uint32_t y = (d & 0x3F3F3F3Fu) | 0x80808080u;
     uint32_t v = 0;

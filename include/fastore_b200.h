@@ -51,7 +51,7 @@ enum { FSB_QUA_NONE = 0, FSB_QUA_BINARY = 1, FSB_QUA_8BIN = 2, FSB_QUA_QVZ = 3 }
 
 /*
  * Binning parameters: the subset of BinModuleConfig (Params.h:167-193) the path reads.
- *   signature_len              MinimizerParameters::signatureLen      (-p, 1..15)
+ *   signature_len              MinimizerParameters::signatureLen      (-p, 3..15)
  *   skip_zone_len              MinimizerParameters::skipZoneLen       (-s)
  *   signature_mask_cutoff_bits MinimizerParameters::signatureMaskCutoffBits (no CLI flag, 0)
  *   paired_end                 ArchiveType::readType == READ_PE       (-z)
