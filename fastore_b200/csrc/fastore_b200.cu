@@ -213,6 +213,7 @@ struct Batch
 {
     bool staged = false, ran = false;
     uint32_t n_chunks = 0;
+    uint32_t chunk0 = 0;                         // index of the first chunk in the caller's list: rejections name the caller's chunk
     uint64_t n_records = 0;
     std::vector<uint64_t> chunk_first_rec;       // n_chunks + 1
     std::vector<uint64_t> chunk_text_base[2], chunk_text_size[2];
@@ -708,7 +709,7 @@ int stage_advance(fsb_ctx* c, Batch& b, cudaStream_t st)
         {
             const ParseSeg& sg = b.segs_host[k];
             if (res[k].first_invalid < b.chunk_n[sg.chunk])
-                return fail(c, FSB_ERR_INPUT, "fsb_stage: record " + std::to_string(res[k].first_invalid) + " of chunk " + std::to_string(sg.chunk) +
+                return fail(c, FSB_ERR_INPUT, "fsb_stage: record " + std::to_string(res[k].first_invalid) + " of chunk " + std::to_string(b.chunk0 + sg.chunk) +
                                                   " is outside the input contract (read length 1..255, title at most 255 bytes)");
         }
         // the tables were written at capacity positions: close the gaps a chunk with fewer records than candidates leaves behind
@@ -737,7 +738,7 @@ int stage_advance(fsb_ctx* c, Batch& b, cudaStream_t st)
 // (records == NULL) are parsed on the device first (parse_enqueue_count here, then stage_advance until b.parse_state is 0).
 // The batch's input buffers must not be in use.  `split` = sub-batches of whole chunks the kernels will run as.  The pipeline
 // keeps its copy stream free of kernels, so that the next sub-batch's text follows at once.
-int stage_enqueue(fsb_ctx* c, Batch& b, const fsb_chunk* chunks, uint32_t n_chunks, cudaStream_t st, cudaStream_t st_check, uint32_t split, bool profile = false)
+int stage_enqueue(fsb_ctx* c, Batch& b, const fsb_chunk* chunks, uint32_t n_chunks, uint32_t chunk0, cudaStream_t st, cudaStream_t st_check, uint32_t split, bool profile = false)
 {
     b.staged = false; b.ran = false; b.parse_state = 0; b.up_used = 0;
     b.split = split; b.profile_check = profile;
@@ -747,6 +748,7 @@ int stage_enqueue(fsb_ctx* c, Batch& b, const fsb_chunk* chunks, uint32_t n_chun
     if (n_chunks > max_chunks) return fail(c, FSB_ERR_PARAM, "fsb_stage: too many chunks in one batch for this signature length (max " + std::to_string(max_chunks) + ")");
 
     b.n_chunks = n_chunks;
+    b.chunk0 = chunk0;
     b.device_parse = chunks[0].records[0] == nullptr && chunks[0].text[0] != nullptr;
     size_t text_bytes[2] = {kTextPad, kTextPad};
     for (int m = 0; m < 2; ++m) { b.chunk_text_base[m].assign(n_chunks, 0); b.chunk_text_size[m].assign(n_chunks, 0); }
@@ -813,7 +815,7 @@ int stage_complete(fsb_ctx* c, Batch& b)
         // never run the kernels on tables that point outside the staged text
         uint32_t ci = 0;
         while (ci + 1 < n_chunks && b.chunk_first_rec[ci + 1] <= stats.first_bad) ++ci;
-        return fail(c, FSB_ERR_INPUT, "fsb_stage: record " + std::to_string(stats.first_bad - b.chunk_first_rec[ci]) + " of chunk " + std::to_string(ci) +
+        return fail(c, FSB_ERR_INPUT, "fsb_stage: record " + std::to_string(stats.first_bad - b.chunk_first_rec[ci]) + " of chunk " + std::to_string(b.chunk0 + ci) +
                                           " violates the input contract (length 1..255, offsets inside the chunk, equal PE mate lengths); " +
                                           std::to_string(stats.n_bad) + " such record(s)");
     }
@@ -821,7 +823,7 @@ int stage_complete(fsb_ctx* c, Batch& b)
     {
         uint32_t ci = 0;
         while (ci + 1 < n_chunks && b.chunk_first_rec[ci + 1] <= stats.first_bad_text) ++ci;
-        return fail(c, FSB_ERR_INPUT, "fsb_stage: record " + std::to_string(stats.first_bad_text - b.chunk_first_rec[ci]) + " of chunk " + std::to_string(ci) +
+        return fail(c, FSB_ERR_INPUT, "fsb_stage: record " + std::to_string(stats.first_bad_text - b.chunk_first_rec[ci]) + " of chunk " + std::to_string(b.chunk0 + ci) +
                                           " holds a byte outside the input contract (sequence symbols A C G T N, quality in [offset, offset + 64), 7-bit title characters); " +
                                           std::to_string(stats.n_bad_text) + " such mate(s)");
     }
@@ -1247,6 +1249,8 @@ extern "C" int fsb_create(const fsb_params* p, int device, void* cuda_stream, fs
     if (std::memcmp(p->dna_symbol_order, "ACGTN", 5) != 0) return fail(nullptr, FSB_ERR_PARAM, "only dna_symbol_order \"ACGTN\" is supported");
     if (p->quality_method > FSB_QUA_QVZ) return fail(nullptr, FSB_ERR_PARAM, "quality_method must be 0..3");
     if (p->quality_method == FSB_QUA_BINARY && p->binary_threshold >= 64) return fail(nullptr, FSB_ERR_PARAM, "binary_threshold must be < 64");
+    // the byte check and the quality coding work on q - offset per byte with bit 7 as a borrow guard (stage_core.cuh, pack_core.cuh)
+    if (p->quality_offset > 127) return fail(nullptr, FSB_ERR_PARAM, "quality_offset must be in [0, 127]");
 
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
@@ -1407,7 +1411,7 @@ extern "C" int fsb_stage(fsb_ctx* c, const fsb_chunk* chunks, uint32_t n_chunks)
     CUDA_TRY(c, cudaSetDevice(c->device));
     CUDA_TRY(c, cudaStreamSynchronize(c->stream));               // nothing may still be using the batch's buffers
     Batch& b = c->batch[0];
-    int rc = stage_enqueue(c, b, chunks, n_chunks, c->stream, c->stream, c->run_split, c->profile);
+    int rc = stage_enqueue(c, b, chunks, n_chunks, 0, c->stream, c->stream, c->run_split, c->profile);
     while (rc == FSB_OK && b.parse_state) rc = stage_advance(c, b, c->stream);      // device-side parse: two more steps, each sized by the one before
     if (rc != FSB_OK) return rc;
     CUDA_TRY(c, cudaStreamSynchronize(c->stream));               // pageable user buffers must outlive the copies; the statistics are back
@@ -1602,7 +1606,7 @@ extern "C" int fsb_bin_chunks(fsb_ctx* c, const fsb_chunk* chunks, uint32_t n_ch
     c->rec_index.assign(c->keep_records ? n_chunks : 0, fsb_ctx::RecRef{{nullptr, nullptr}, 0});
 
     for (uint32_t g = 0; g < std::min(G, kAhead) && rc == FSB_OK; ++g)
-        rc = stage_enqueue(c, set_of(g), chunks + first[g], first[g + 1] - first[g], c->s_h2d, c->s_chk[g % kSets], 1);
+        rc = stage_enqueue(c, set_of(g), chunks + first[g], first[g + 1] - first[g], first[g], c->s_h2d, c->s_chk[g % kSets], 1);
     trace.mark("first copies enqueued", 0);
     for (uint32_t g = 0; g < G && rc == FSB_OK; ++g)
     {
@@ -1623,7 +1627,7 @@ extern "C" int fsb_bin_chunks(fsb_ctx* c, const fsb_chunk* chunks, uint32_t n_ch
         // starts the moment they end -- the host has nothing else to do until the text of g+1 has arrived.
         if (g + kAhead < G)
         {
-            if ((rc = stage_enqueue(c, set_of(g + kAhead), chunks + first[g + kAhead], first[g + kAhead + 1] - first[g + kAhead], c->s_h2d, c->s_chk[(g + kAhead) % kSets], 1)) != FSB_OK) break;
+            if ((rc = stage_enqueue(c, set_of(g + kAhead), chunks + first[g + kAhead], first[g + kAhead + 1] - first[g + kAhead], first[g + kAhead], c->s_h2d, c->s_chk[(g + kAhead) % kSets], 1)) != FSB_OK) break;
         }
         if ((rc = finish(g)) != FSB_OK) break;
         trace.mark("copy out enqueued", g);

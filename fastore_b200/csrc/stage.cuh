@@ -9,6 +9,7 @@
 #include <cuda_runtime.h>
 
 #include "core.cuh"
+#include "stage_core.cuh"
 
 namespace fsb {
 
@@ -90,68 +91,12 @@ __global__ void __launch_bounds__(256) stage_stats_kernel(BatchView B, DevicePar
 // parser applies (csrc/host/fastq_parser.cpp).  It is a streaming pass over the staged text with 16-byte loads
 // (a half warp per mate: lane j checks the j-th aligned 16-byte piece of the sequence, of the quality and of the
 // title), part of fsb_stage, not of the timed fsb_run path.
-// 0xFF for every byte of a 4-byte word whose offset word_base + b lies in [lo, hi)
-__device__ __forceinline__ uint32_t bytes_in_range_mask(int32_t lo, int32_t hi, int32_t word_base)
-{
-    const int32_t a = min(max(lo - word_base, 0), 4), b = min(max(hi - word_base, 0), 4);      // bytes [a, b) of the word
-    uint32_t ma, mb;                                                                          // shl.b32 clamps counts above 31 (result 0)
-    asm("shl.b32 %0, %1, %2;" : "=r"(ma) : "r"(0xFFFFFFFFu), "r"(8u * (uint32_t)a));
-    asm("shl.b32 %0, %1, %2;" : "=r"(mb) : "r"(0xFFFFFFFFu), "r"(8u * (uint32_t)b));
-    return ma & ~mb;
-}
-// All four bytes at once.  A valid base is one of A 0x41, C 0x43, G 0x47, T 0x54, N 0x4E: bits 7..5 are 010, and with
-// c = bits 3..1 (the code K1's bit planes are built from: A 000, C 001, T 010, G 011, N 111; 100, 101, 110 do not
-// occur) bit 4 is set for T only and bit 0 is clear for T and N only.  Bit k of every byte is looked at in place
-// (w >> k keeps it at bit 0 of the byte; the other bits of the byte are masked off at the end).
-__device__ __forceinline__ bool dna_word_ok(uint32_t w, uint32_t m)
-{
-    w = (w & m) | (0x41414141u & ~m);                                 // bytes outside the span count as 'A'
-    const uint32_t s1 = w >> 1, s2 = w >> 2, s3 = w >> 3, s4 = w >> 4, s5 = w >> 5;
-    const uint32_t isT = ~s3 & s2 & ~s1, isN = s3 & s2 & s1;
-    const uint32_t bad_code = s3 & ~(s2 & s1);
-    const uint32_t bad_b4 = s4 ^ isT, bad_b0 = w ^ ~(isT | isN);
-    const uint32_t low = (bad_code | bad_b4 | bad_b0) & 0x01010101u;
-    const uint32_t high = (s5 ^ 0x02020202u) & 0x07070707u;
-    return (low | high) == 0;
-}
-// q - offset in [0, 64) for the 6- and 3-bit modes (need_range), q >= offset for the 1-bit mode; off4 = offset * 0x01010101, offset <= 127.
-// Per byte t = (q | 128) - offset never borrows from its neighbour.  For q < 128 that is q - offset + 128: in range <=> bit 7 set and
-// bit 6 clear; for q >= 128 it is q - offset itself: in range <=> bits 7 and 6 clear.
-__device__ __forceinline__ bool qua_word_ok(uint32_t w, uint32_t m, uint32_t off4, bool need_range)
-{
-    w = (w & m) | (off4 & ~m);                                        // bytes outside the span count as quality 0
-    const uint32_t t = (w | 0x80808080u) - off4;
-    const uint32_t h = w & 0x80808080u;
-    const uint32_t bad = need_range ? ((t ^ ~h) | (t << 1)) : (~t & ~w);
-    return (bad & 0x80808080u) == 0;
-}
-
-// one aligned 16-byte piece of a span: `lo`/`hi` = the span's byte range counted from the aligned address a0
-template <int KIND>     // 0 sequence, 1 quality, 2 title characters
+// The checks of one piece live in stage_core.cuh; here the piece arrives as one 16-byte load.
+template <int KIND>
 __device__ __forceinline__ bool piece_ok(const uint4& q, int32_t piece, int32_t lo, int32_t hi, uint32_t off4, bool need_range)
 {
     const uint32_t w[4] = {q.x, q.y, q.z, q.w};
-    const bool inner = piece * 16 >= lo && piece * 16 + 16 <= hi;     // every byte of the piece belongs to the span (all but the first and last piece)
-    bool ok = true;
-#pragma unroll
-    for (int j = 0; j < 4; ++j)
-    {
-        const uint32_t msk = inner ? 0xFFFFFFFFu : bytes_in_range_mask(lo, hi, piece * 16 + 4 * j);
-        if (KIND == 0) ok = ok && dna_word_ok(w[j], msk);
-        else if (KIND == 1) ok = ok && qua_word_ok(w[j], msk, off4, need_range);
-        else ok = ok && ((w[j] & msk & 0x80808080u) == 0);
-    }
-    return ok;
-}
-
-struct CheckSpan { uintptr_t a0; int32_t lo, hi; };
-__device__ __forceinline__ CheckSpan check_span(const uint8_t* p0, uint32_t len)
-{
-    CheckSpan s;
-    s.a0 = reinterpret_cast<uintptr_t>(p0) & ~(uintptr_t)15;          // the text buffers are padded: aligned pieces stay inside
-    s.lo = (int32_t)(reinterpret_cast<uintptr_t>(p0) - s.a0);
-    s.hi = len ? s.lo + (int32_t)len : 0;                             // hi = 0: nothing to check
-    return s;
+    return piece_ok<KIND>(w, piece, lo, hi, off4, need_range);
 }
 
 // A half warp per mate: lane j checks the j-th aligned 16-byte piece of the sequence, of the quality and of the title (the
@@ -176,7 +121,7 @@ __global__ void __launch_bounds__(256) validate_text_kernel(BatchView B, DeviceP
     const int32_t l16 = (int32_t)(threadIdx.x & 15u);
     const uint64_t n_mates = P.paired ? 2 * B.n_records : B.n_records;
     const bool need_range = P.qua_bits != 1;                                            // 1-bit mode: only q >= offset (the threshold compare takes any value)
-    const uint32_t off4 = (P.qua_offset & 0x7Fu) * 0x01010101u;
+    const uint32_t off4 = quality_off4(P.qua_offset);
     const uint64_t stride = (uint64_t)gridDim.x * 16u;
     uint64_t g = (uint64_t)blockIdx.x * 16u + half;
     auto load_rec = [&](uint64_t gg) -> uint4

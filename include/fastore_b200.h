@@ -56,7 +56,7 @@ enum { FSB_QUA_NONE = 0, FSB_QUA_BINARY = 1, FSB_QUA_8BIN = 2, FSB_QUA_QVZ = 3 }
  *   signature_mask_cutoff_bits MinimizerParameters::signatureMaskCutoffBits (no CLI flag, 0)
  *   paired_end                 ArchiveType::readType == READ_PE       (-z)
  *   quality_method             QualityCompressionParams::method       (-q0..3)
- *   quality_offset             ArchiveType::qualityOffset             (33, or 64 with -I)
+ *   quality_offset             ArchiveType::qualityOffset             (0..127: 33, or 64 with -I)
  *   binary_threshold           QualityCompressionParams::binaryThreshold (-w, default 20)
  *   reads_have_headers         ArchiveType::readsHaveHeaders          (-H)
  *   dna_symbol_order           MinimizerParameters::dnaSymbolOrder    (only "ACGTN" is accepted)

@@ -482,3 +482,49 @@ extern "C" uint64_t emul_parse_text(const uint8_t* text, uint64_t size, int keep
     }
     return n;
 }
+
+// ---- FSB_OPT_VALIDATE: validate_text_kernel's per-mate byte check (stage_core.cuh) -------------------------------------
+// `spans` holds n triples (offset into buf, length, kind: 0 sequence, 1 quality, 2 title characters).  buf is copied to a
+// 16-byte aligned buffer with 64 zero bytes behind it, so the aligned pieces stay inside as they do in the padded device
+// text.  Each span is checked the way one half warp checks a mate: lanes 0..15 take pieces 0..15, then each lane its
+// pieces 16, 32, ... (the 17th piece of spans over 240 bytes).  ok[i] = 1 when span i passes.
+#include "../../fastore_b200/csrc/stage_core.cuh"
+
+extern "C" void emul_check_spans(const uint8_t* buf, uint64_t size, const int32_t* spans, uint64_t n, uint32_t qua_offset, int need_range, uint8_t* ok)
+{
+    struct alignas(16) Piece { uint8_t b[16]; };
+    std::vector<Piece> text((size + 64 + 15) / 16);
+    std::memset(text.data(), 0, text.size() * sizeof(Piece));
+    std::memcpy(text.data(), buf, size);
+    const uint8_t* base = text.data()->b;
+    const uint32_t off4 = fsb::quality_off4(qua_offset);
+    for (uint64_t i = 0; i < n; ++i)
+    {
+        const int32_t kind = spans[3 * i + 2];
+        const CheckSpan s = check_span(base + spans[3 * i], (uint32_t)spans[3 * i + 1]);
+        auto piece = [&](int32_t p) {
+            uint32_t w[4];
+            std::memcpy(w, reinterpret_cast<const uint8_t*>(s.a0) + 16 * p, 16);
+            return kind == 0 ? piece_ok<0>(w, p, s.lo, s.hi, off4, need_range != 0)
+                 : kind == 1 ? piece_ok<1>(w, p, s.lo, s.hi, off4, need_range != 0)
+                             : piece_ok<2>(w, p, s.lo, s.hi, off4, need_range != 0);
+        };
+        bool all = true;
+        for (int32_t l16 = 0; l16 < 16; ++l16)
+        {
+            bool lane = true;
+            if (l16 * 16 < s.hi) lane = piece(l16);
+            for (int32_t p = l16 + 16; p * 16 < s.hi; p += 16) lane = lane && piece(p);
+            all = all && lane;
+        }
+        ok[i] = all ? 1 : 0;
+    }
+}
+
+// quality4<Q> (pack_core.cuh) on single words, with off4 / thr4 formed as pack_quality_to forms them
+extern "C" void emul_quality4(int q_bits, const uint32_t* words, uint64_t n, uint32_t qua_offset, uint32_t threshold, uint32_t* out)
+{
+    const uint32_t off4 = qua_offset * 0x01010101u, thr4 = threshold * 0x01010101u;
+    for (uint64_t i = 0; i < n; ++i)
+        out[i] = q_bits == 6 ? quality4<6>(words[i], off4, thr4) : q_bits == 3 ? quality4<3>(words[i], off4, thr4) : quality4<1>(words[i], off4, thr4);
+}
