@@ -994,7 +994,8 @@ int run_sub(fsb_ctx* c, Batch& b, const Sub& sb, fsb_ctx::Lane& L, cudaEvent_t* 
             const bool count_next = c->fused_hist && pass + 1 < passes;
             const uint32_t next_radix = count_next ? (1u << width[pass + 1]) : 0u;
             if (count_next) CUDA_TRY(c, cudaMemsetAsync(L.d_counts.p, 0, (size_t)next_radix * nblocks * 4, st));
-            sort_scatter<<<nblocks, kSortThreads, 0, st>>>(L.d_keys[cur].as<uint32_t>(), L.d_cards[cur].as<unsigned long long>(), tiles, shift, mask, radix,
+            CUDA_TRY(c, cudaFuncSetAttribute(sort_scatter, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SortScatterSmem)));
+            sort_scatter<<<nblocks, kSortThreads, sizeof(SortScatterSmem), st>>>(L.d_keys[cur].as<uint32_t>(), L.d_cards[cur].as<unsigned long long>(), tiles, shift, mask, radix,
                                                             L.d_counts_scan.as<uint32_t>(), L.d_keys[cur ^ 1].as<uint32_t>(), L.d_cards[cur ^ 1].as<unsigned long long>(),
                                                             count_next ? L.d_counts.as<uint32_t>() : nullptr, shift + width[pass], next_radix ? next_radix - 1u : 0u, next_radix);
             counted = count_next;
@@ -1026,11 +1027,13 @@ int run_sub(fsb_ctx* c, Batch& b, const Sub& sb, fsb_ctx::Lane& L, cudaEvent_t* 
         const unsigned nlay = (unsigned)((n + kLayBlock - 1) / kLayBlock);
         LayState* states = L.d_lay_states.as<LayState>();
         ChunkStart* cstart = L.d_chunk_start.as<ChunkStart>();
-        lay_reduce_kernel<<<nlay, kLayThreads, 0, st>>>(n, P, S, b.min_len, states);
+        CUDA_TRY(c, cudaFuncSetAttribute(lay_reduce_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLayReduceSmem));
+        CUDA_TRY(c, cudaFuncSetAttribute(lay_apply_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLayApplySmem));
+        lay_reduce_kernel<<<nlay, kLayThreads, kLayReduceSmem, st>>>(n, P, S, b.min_len, states);
         const unsigned ngroups = (nlay + kLayScanThreads - 1) / kLayScanThreads;
         lay_scan_groups_kernel<<<ngroups, kLayScanThreads, 0, st>>>(states, nlay, states + nlay + 1);
         lay_scan_finish_kernel<<<ngroups, kLayScanThreads, 0, st>>>(states, nlay, states + nlay + 1);
-        lay_apply_kernel<<<nlay, kLayThreads, 0, st>>>(n, sub_chunks, P, S, b.min_len, states, LayOut{pm, O, desc, cstart, L.d_nb.as<uint32_t>()});
+        lay_apply_kernel<<<nlay, kLayThreads, kLayApplySmem, st>>>(n, sub_chunks, P, S, b.min_len, states, LayOut{pm, O, desc, cstart, L.d_nb.as<uint32_t>()});
         chunk_summary_fused_kernel<<<sub_chunks, 128, 0, st>>>(B, cstart, desc, b.d_summary.as<ChunkSummary>() + sb.c0);
         launches += 5;
     }

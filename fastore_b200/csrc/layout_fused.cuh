@@ -6,7 +6,9 @@
 // plus the bin descriptors and the per-chunk summary.  The arithmetic is layout_core.cuh's scan.
 //
 // Mapping: a thread owns one K4 tile (32 consecutive sorted records) and walks over it sequentially; a block
-// of 128 threads owns 4096 records.
+// of 128 threads owns 4096 records.  A warp first copies its 32 runs into shared memory with coalesced loads (a
+// thread's own 128 + 256 contiguous bytes, loaded by the thread, would touch 32 lines per warp instruction), and
+// lay_apply stages loc / binfo in shared memory for eight records a round so that the warp writes whole sectors.
 //   lay_reduce   every block's LayState                              -> tile_states[block]
 //   lay_scan_groups / lay_scan_finish   exclusive scan over the block states (in place; [nblocks] = the whole batch)
 //   lay_apply    thread prefix = block prefix (+) threads in front; absolute walk that writes loc / binfo / tbase,
@@ -25,7 +27,7 @@ namespace fsb {
 constexpr uint32_t kLayThreads = 128;
 constexpr uint32_t kLayPerThread = kPlaceTile;                      // a thread walks over one K4 tile
 constexpr uint32_t kLayBlock = kLayThreads * kLayPerThread;         // 4096 records per block
-static_assert(kLayPerThread == 32, "lay_apply stores a thread's values as 16-byte vectors of four");
+static_assert(kLayPerThread == 32, "a warp stages its runs as 32 x 32 records");
 
 // ---- moving a LayState between lanes ---------------------------------------------------------------------------
 constexpr int kLayWords = (int)(sizeof(LayState) / 4);
@@ -85,47 +87,86 @@ __device__ __forceinline__ LayRun lay_run(uint64_t n)
     r.cnt = r.i0 < n ? (uint32_t)min((uint64_t)kLayPerThread, n - r.i0) : 0u;
     return r;
 }
-// the state of a thread's run (keys and cards are read as 16-byte vectors: the run is 128 / 256 contiguous bytes)
-__device__ __forceinline__ LayState lay_run_state(const DeviceParams& P, const SortedView& S, const LayRun& run, uint32_t uniform_len)
+
+// A warp's 32 runs in shared memory, one row per thread.  Rows of 33 entries: a thread walking its row and the
+// warp filling the rows with coalesced loads both hit 32 different banks.
+constexpr uint32_t kLayRow = kLayPerThread + 1;
+struct LayWarpIn
 {
-    LayState st = lay_identity();
-    if (run.cnt == 0) return st;
-    uint32_t prev = run.i0 ? S.skeys[run.i0 - 1] : 0u;
-    if (run.cnt == kLayPerThread)
+    uint32_t keys[32][kLayRow];
+    unsigned long long cards[32][kLayRow];
+};
+// loc[0..3] and binfo of one round of kLayRound records per thread, before the warp writes them out together
+constexpr uint32_t kLayRound = 8;
+constexpr uint32_t kLayOutWords = 5 * 32 * kLayRound;
+constexpr size_t kLayReduceSmem = (kLayThreads / 32) * sizeof(LayWarpIn);
+constexpr size_t kLayApplySmem = (kLayThreads / 32) * (sizeof(LayWarpIn) + kLayOutWords * 4);
+static_assert(sizeof(LayWarpIn) % 16 == 0, "the out staging behind the runs takes 16-byte vectors");
+
+// the records [wb, wb + 32 * kLayPerThread) of the warp (those below n) into its rows, with 16-byte loads
+__device__ __forceinline__ void lay_stage(const SortedView& S, uint64_t n, uint64_t wb, LayWarpIn& w)
+{
+    const unsigned lane = threadIdx.x & 31;
+    if (wb + 32 * kLayPerThread <= n)
     {
-        const uint4* k4 = reinterpret_cast<const uint4*>(S.skeys + run.i0);
-        const ulonglong2* c2 = reinterpret_cast<const ulonglong2*>(S.cards + run.i0);
-#pragma unroll 2
-        for (uint32_t q = 0; q < kLayPerThread / 4; ++q)
-        {
-            const uint4 kk = k4[q];
-            const ulonglong2 ca = c2[2 * q], cb = c2[2 * q + 1];
-            const uint32_t key[4] = {kk.x, kk.y, kk.z, kk.w};
-            const unsigned long long card[4] = {ca.x, ca.y, cb.x, cb.y};
+        const uint4* k4 = reinterpret_cast<const uint4*>(S.skeys + wb);
+        const ulonglong2* c2 = reinterpret_cast<const ulonglong2*>(S.cards + wb);
 #pragma unroll
-            for (int u = 0; u < 4; ++u)
-            {
-                lay_push(st, lay_record(P, run.i0 + 4 * q + u == 0, key[u], prev, card[u], uniform_len));
-                prev = key[u];
-            }
+        for (uint32_t it = 0; it < kLayPerThread / 4; ++it)
+        {
+            const uint32_t v = it * 32 + lane;
+            const uint4 q = k4[v];
+            uint32_t* o = &w.keys[v / 8][4 * (v % 8)];
+            o[0] = q.x; o[1] = q.y; o[2] = q.z; o[3] = q.w;
+        }
+#pragma unroll
+        for (uint32_t it = 0; it < kLayPerThread / 2; ++it)
+        {
+            const uint32_t v = it * 32 + lane;
+            const ulonglong2 q = c2[v];
+            unsigned long long* o = &w.cards[v / 16][2 * (v % 16)];
+            o[0] = q.x; o[1] = q.y;
         }
     }
     else
     {
-        for (uint32_t j = 0; j < run.cnt; ++j)
+        for (uint32_t r = lane; r < 32 * kLayPerThread && wb + r < n; r += 32)
         {
-            const uint32_t key = S.skeys[run.i0 + j];
-            lay_push(st, lay_record(P, run.i0 + j == 0, key, prev, S.cards[run.i0 + j], uniform_len));
-            prev = key;
+            w.keys[r / kLayPerThread][r % kLayPerThread] = S.skeys[wb + r];
+            w.cards[r / kLayPerThread][r % kLayPerThread] = S.cards[wb + r];
         }
+    }
+    __syncwarp();
+}
+// the key in front of the thread's run (only the last run of a batch is partial, so the run in front is whole)
+__device__ __forceinline__ uint32_t lay_prev_key(const SortedView& S, const LayWarpIn& w, const LayRun& run)
+{
+    const unsigned lane = threadIdx.x & 31;
+    return lane ? w.keys[lane - 1][kLayPerThread - 1] : (run.i0 ? S.skeys[run.i0 - 1] : 0u);
+}
+// the state of a thread's run, walked from its row
+__device__ __forceinline__ LayState lay_run_state(const DeviceParams& P, const LayWarpIn& w, uint32_t prev, const LayRun& run, uint32_t uniform_len)
+{
+    const unsigned lane = threadIdx.x & 31;
+    LayState st = lay_identity();
+#pragma unroll 4
+    for (uint32_t j = 0; j < run.cnt; ++j)
+    {
+        const uint32_t key = w.keys[lane][j];
+        lay_push(st, lay_record(P, run.i0 + j == 0, key, prev, w.cards[lane][j], uniform_len));
+        prev = key;
     }
     return st;
 }
 
 __global__ void __launch_bounds__(kLayThreads) lay_reduce_kernel(uint64_t n, DeviceParams P, SortedView S, uint32_t uniform_len, LayState* __restrict__ tile_states)
 {
+    extern __shared__ uint4 lay_smem_raw[];
     __shared__ LayState sm[kLayThreads / 32];
-    const LayState mine = lay_run_state(P, S, lay_run(n), uniform_len);
+    LayWarpIn& w = reinterpret_cast<LayWarpIn*>(lay_smem_raw)[threadIdx.x >> 5];
+    const LayRun run = lay_run(n);
+    lay_stage(S, n, run.i0 - (uint64_t)(threadIdx.x & 31) * kLayPerThread, w);
+    const LayState mine = lay_run_state(P, w, lay_prev_key(S, w, run), run, uniform_len);
     LayState total;
     lay_block_scan(mine, total, sm);
     if (threadIdx.x == 0) tile_states[blockIdx.x] = total;
@@ -186,50 +227,45 @@ struct LayOut
 __global__ void __launch_bounds__(kLayThreads) lay_apply_kernel(uint64_t n, uint32_t n_chunks, DeviceParams P, SortedView S, uint32_t uniform_len,
                                                                 const LayState* __restrict__ tile_prefix, LayOut out)
 {
+    extern __shared__ uint4 lay_smem_raw[];
     __shared__ LayState sm[kLayThreads / 32];
+    const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    LayWarpIn& w = reinterpret_cast<LayWarpIn*>(lay_smem_raw)[warp];
+    // per array (loc[0..3], binfo) and thread: two 16-byte halves of a round, swapped in every other group of four
+    // threads so that neither the threads' stores nor the warp's loads meet twice in a bank
+    uint4* ost = reinterpret_cast<uint4*>(reinterpret_cast<LayWarpIn*>(lay_smem_raw) + kLayThreads / 32) + warp * (kLayOutWords / 4);
     const LayRun run = lay_run(n);
-    const LayState mine = lay_run_state(P, S, run, uniform_len);
+    const uint64_t wb = run.i0 - (uint64_t)lane * kLayPerThread;   // the warp's first record
+    lay_stage(S, n, wb, w);
+    uint32_t prev = lay_prev_key(S, w, run);
+    const LayState mine = lay_run_state(P, w, prev, run, uniform_len);
     LayState total;
     const LayState excl = lay_combine(tile_prefix[blockIdx.x], lay_block_scan(mine, total, sm));
-    if (run.cnt == 0) return;
     LayCursor cur = lay_cursor(excl);
     const uint64_t tile = run.i0 / kPlaceTile;                      // the thread's K4 tile
     const uint32_t key_mask = (1u << P.key_bits) - 1u;
     const bool has_head = P.has_headers != 0;
-    uint32_t prev = run.i0 ? S.skeys[run.i0 - 1] : 0u;
+    // the key behind the run
+    const uint32_t key_after = lane < 31 ? w.keys[lane + 1][0] : (run.i0 + kLayPerThread < n ? S.skeys[run.i0 + kLayPerThread] : 0u);
     unsigned long long b0[4] = {0, 0, 0, 0};                        // first bit of the tile in every stream
     uint32_t base_bits_lo[4] = {0, 0, 0, 0};
-    uint32_t loc[4][4], binfo[4];
-    for (uint32_t q = 0; 4u * q < run.cnt; ++q)
+    for (uint32_t rnd = 0; rnd < kLayPerThread / kLayRound; ++rnd)
     {
-        // the round's four keys and cards as vectors (a warp-wide scalar load here would touch 32 lines for 4 bytes each)
-        uint32_t gk[4] = {0, 0, 0, 0};
-        unsigned long long gc[4] = {0, 0, 0, 0};
-        if (4u * q + 4u <= run.cnt)
-        {
-            const uint4 kk = *reinterpret_cast<const uint4*>(S.skeys + run.i0 + 4u * q);
-            const ulonglong2 ca = *reinterpret_cast<const ulonglong2*>(S.cards + run.i0 + 4u * q), cb = *reinterpret_cast<const ulonglong2*>(S.cards + run.i0 + 4u * q + 2u);
-            gk[0] = kk.x; gk[1] = kk.y; gk[2] = kk.z; gk[3] = kk.w;
-            gc[0] = ca.x; gc[1] = ca.y; gc[2] = cb.x; gc[3] = cb.y;
-        }
-        else
-        {
+        uint32_t loc[4][kLayRound], binfo[kLayRound];
 #pragma unroll
-            for (int u = 0; u < 4; ++u) if (4u * q + (uint32_t)u < run.cnt) { gk[u] = S.skeys[run.i0 + 4u * q + u]; gc[u] = S.cards[run.i0 + 4u * q + u]; }
-        }
-        const uint64_t after = run.i0 + 4u * q + 4u;                  // the record behind the round
-        const uint32_t key_after = (4u * q + 4u <= run.cnt && after < n) ? S.skeys[after] : 0u;
-#pragma unroll
-        for (int u = 0; u < 4; ++u)                                   // four records per round: their values leave as one 16-byte vector per array
+        for (uint32_t u = 0; u < kLayRound; ++u)
         {
-            const uint32_t j = 4u * q + (uint32_t)u;
+            const uint32_t j = rnd * kLayRound + u;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) loc[k][u] = 0;
+            binfo[u] = 0;
             if (j < run.cnt)
             {
                 const uint64_t i = run.i0 + j;
-                const uint32_t key = gk[u];
+                const uint32_t key = w.keys[lane][j];
                 // the key behind this record; the last record of the batch closes its bin whatever follows
-                const uint32_t next = i + 1 >= n ? ~key : (u < 3 ? gk[(u + 1) & 3] : key_after);
-                const LayRec r = lay_record(P, i == 0, key, prev, gc[u], uniform_len);
+                const uint32_t next = i + 1 >= n ? ~key : (j + 1 < kLayPerThread ? w.keys[lane][j + 1] : key_after);
+                const LayRec r = lay_record(P, i == 0, key, prev, w.cards[lane][j], uniform_len);
                 uint64_t at[4];
                 lay_step(cur, r, at);
                 if (r.chunk_start)
@@ -263,26 +299,42 @@ __global__ void __launch_bounds__(kLayThreads) lay_apply_kernel(uint64_t n, uint
                 prev = key;
             }
         }
-        const uint64_t g = run.i0 + 4u * q;                           // first record of the group of four
-        if (4u * q + 4u <= run.cnt)
-        {
+        const uint32_t sw = (lane >> 2) & 1u;
 #pragma unroll
-            for (int k = 0; k < 4; ++k) *reinterpret_cast<uint4*>(out.pm.loc[k] + g) = make_uint4(loc[k][0], loc[k][1], loc[k][2], loc[k][3]);
-            *reinterpret_cast<uint4*>(out.pm.binfo + g) = make_uint4(binfo[0], binfo[1], binfo[2], binfo[3]);
+        for (int k = 0; k < 4; ++k)
+        {
+            ost[(k * 32 + lane) * 2 + sw] = make_uint4(loc[k][0], loc[k][1], loc[k][2], loc[k][3]);
+            ost[(k * 32 + lane) * 2 + (sw ^ 1u)] = make_uint4(loc[k][4], loc[k][5], loc[k][6], loc[k][7]);
         }
-        else
-        {
+        ost[(4 * 32 + lane) * 2 + sw] = make_uint4(binfo[0], binfo[1], binfo[2], binfo[3]);
+        ost[(4 * 32 + lane) * 2 + (sw ^ 1u)] = make_uint4(binfo[4], binfo[5], binfo[6], binfo[7]);
+        __syncwarp();
+        // the warp writes the round out: two lanes per thread, 32 contiguous bytes per thread and array
 #pragma unroll
-            for (int v = 0; v < 3; ++v)
-                if (4u * q + (uint32_t)v < run.cnt)
+        for (uint32_t it = 0; it < 2; ++it)
+        {
+            const uint32_t t = it * 16 + (lane >> 1), h = lane & 1u;
+            const uint64_t g = wb + (uint64_t)t * kLayPerThread + rnd * kLayRound + 4 * h;
+            if (g < n)
+            {
+#pragma unroll
+                for (int a = 0; a < 5; ++a)
                 {
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) out.pm.loc[k][g + v] = loc[k][v];
-                    out.pm.binfo[g + v] = binfo[v];
+                    const uint4 q = ost[(a * 32 + t) * 2 + (h ^ ((t >> 2) & 1u))];
+                    uint32_t* dst = a < 4 ? out.pm.loc[a] : out.pm.binfo;
+                    if (g + 4 <= n) *reinterpret_cast<uint4*>(dst + g) = q;
+                    else
+                    {
+                        dst[g] = q.x;
+                        if (g + 1 < n) dst[g + 1] = q.y;
+                        if (g + 2 < n) dst[g + 2] = q.z;
+                    }
                 }
+            }
         }
+        __syncwarp();
     }
-    if (run.i0 + run.cnt == n)
+    if (run.cnt && run.i0 + run.cnt == n)
     {   // end of the batch: the end of the last tile, the totals
         const uint64_t tiles = (n + kPlaceTile - 1) / kPlaceTile;
         ChunkStart cs;

@@ -283,43 +283,105 @@ __device__ __forceinline__ uint64_t sort_count_index(const SortTile& t, uint32_t
     return (uint64_t)radix * t.cblk + (uint64_t)digit * t.nblk + t.blk;
 }
 
+// A tile's keys or cards as 16-byte vectors: [0, head) and [head + nvec * PER, count) are read one by one, the
+// vectors in between start at a 16-byte boundary (the tiles of a chunk start wherever the chunk's records do).
+template <typename T>
+struct TileSplit
+{
+    static constexpr uint32_t PER = 16u / sizeof(T);
+    uint32_t head, nvec;
+    __device__ __forceinline__ TileSplit(const T* src, uint32_t count)
+    {
+        head = min(count, (uint32_t)((16u - (reinterpret_cast<uintptr_t>(src) & 15u)) & 15u) / (uint32_t)sizeof(T));
+        nvec = (count - head) / PER;
+    }
+};
+
+constexpr int kSortWarps = kSortThreads / 32;
+
 __global__ void __launch_bounds__(kSortThreads) sort_histogram(const uint32_t* __restrict__ keys, const SortTile* __restrict__ tiles, int shift, uint32_t mask,
                                                                 uint32_t radix, uint32_t* __restrict__ counts)
 {
-    __shared__ uint32_t hist[kMaxRadix];
-    for (uint32_t d = threadIdx.x; d < radix; d += kSortThreads) hist[d] = 0;
+    __shared__ uint32_t hist[kSortWarps][kMaxRadix];                // one sub-histogram per warp: 16 KB
+    const unsigned warp = threadIdx.x >> 5;
+    for (uint32_t d = threadIdx.x; d < radix; d += kSortThreads)
+#pragma unroll
+        for (int w = 0; w < kSortWarps; ++w) hist[w][d] = 0;
     __syncthreads();
     const SortTile t = tiles[blockIdx.x];
+    const uint32_t* src = keys + t.first;
+    const TileSplit<uint32_t> sp(src, t.count);
+    uint32_t* h = hist[warp];
+    const uint4* v = reinterpret_cast<const uint4*>(src + sp.head);
 #pragma unroll 4
-    for (int i = 0; i < kSortStrips; ++i)
+    for (uint32_t i = threadIdx.x; i < sp.nvec; i += kSortThreads)
     {
-        const uint32_t local = (uint32_t)i * kSortThreads + threadIdx.x;
-        const bool in = local < t.count;
-        const uint32_t d = in ? ((keys[t.first + local] >> shift) & mask) : 0xFFFFFFFFu;
-        // warp-aggregated shared atomics: bins are heavily skewed (minimizers are minima)
-        const unsigned peers = __match_any_sync(0xFFFFFFFFu, d);
-        if (in && (__ffs(peers) - 1) == (int)(threadIdx.x & 31)) atomicAdd(&hist[d], (uint32_t)__popc(peers));
+        const uint4 q = v[i];
+        atomicAdd(&h[(q.x >> shift) & mask], 1u);
+        atomicAdd(&h[(q.y >> shift) & mask], 1u);
+        atomicAdd(&h[(q.z >> shift) & mask], 1u);
+        atomicAdd(&h[(q.w >> shift) & mask], 1u);
     }
+    if (threadIdx.x < sp.head) atomicAdd(&h[(src[threadIdx.x] >> shift) & mask], 1u);
+    const uint32_t tail = sp.head + sp.nvec * 4u + threadIdx.x;
+    if (tail < t.count) atomicAdd(&h[(src[tail] >> shift) & mask], 1u);
     __syncthreads();
-    for (uint32_t d = threadIdx.x; d < radix; d += kSortThreads) counts[sort_count_index(t, radix, d)] = hist[d];
+    for (uint32_t d = threadIdx.x; d < radix; d += kSortThreads)
+    {
+        uint32_t c = 0;
+#pragma unroll
+        for (int w = 0; w < kSortWarps; ++w) c += hist[w][d];
+        counts[sort_count_index(t, radix, d)] = c;
+    }
 }
 
+// Copies a tile's keys or cards into shared memory with 16-byte loads.  `buf` has PER - 1 spare entries: the tile starts at
+// buf + (its misalignment), so that the vectors land on 16-byte boundaries in shared memory too.  Returns the tile's start.
+template <typename T>
+__device__ __forceinline__ T* sort_stage(const T* __restrict__ src, uint32_t count, T* buf)
+{
+    const TileSplit<T> sp(src, count);
+    T* dst = buf + (sp.head ? TileSplit<T>::PER - sp.head : 0u);
+    const uint4* v = reinterpret_cast<const uint4*>(src + sp.head);
+    uint4* o = reinterpret_cast<uint4*>(dst + sp.head);
+    for (uint32_t i = threadIdx.x; i < sp.nvec; i += kSortThreads) o[i] = v[i];
+    if (threadIdx.x < sp.head) dst[threadIdx.x] = src[threadIdx.x];
+    const uint32_t tail = sp.head + sp.nvec * TileSplit<T>::PER + threadIdx.x;
+    if (tail < count) dst[tail] = src[tail];
+    return dst;
+}
+
+// Shared memory of sort_scatter (dynamic: more than the 48 KB a static array may take).
+struct SortScatterSmem
+{
+    unsigned long long cards[kSortTile + 2];   // the tile's cards, then the same cards in (digit, rank) order
+    uint32_t keys[kSortTile + 4];              // the same for the keys
+    uint32_t warp_hist[kSortWarps][kMaxRadix]; // per warp and digit: keys, then the tile-local slot of the warp's first key
+    uint32_t gbase[kMaxRadix];                 // per digit: global destination of tile-local slot 0
+    uint32_t scan[kSortWarps + 1];
+};
+
 // offsets: exclusive scan of counts (same layout).  The 64-bit values are the records' cards (core.cuh).
+// The tile is ranked in shared memory (stable: warp-major, input order inside a warp's strips) and reordered there into
+// (digit, rank) order, so that consecutive threads store consecutive keys of one digit's run.
 // next_counts (may be null): the count table of the NEXT pass, zeroed by the caller -- a key's destination tells the tile it
 // will sit in, so the next pass needs no histogram kernel of its own (one L2 reduction per key, spread over tiles x digits counters).
-// (launch bound of 4 blocks per SM: the kernel lives on scattered stores in flight, not on registers)
-__global__ void __launch_bounds__(kSortThreads, 4) sort_scatter(const uint32_t* __restrict__ keys_in, const unsigned long long* __restrict__ vals_in,
+__global__ void __launch_bounds__(kSortThreads) sort_scatter(const uint32_t* __restrict__ keys_in, const unsigned long long* __restrict__ vals_in,
                                                               const SortTile* __restrict__ tiles, int shift, uint32_t mask, uint32_t radix,
                                                               const uint32_t* __restrict__ offsets, uint32_t* __restrict__ keys_out,
                                                               unsigned long long* __restrict__ vals_out,
                                                               uint32_t* __restrict__ next_counts, int next_shift, uint32_t next_mask, uint32_t next_radix)
 {
-    __shared__ uint32_t warp_hist[kSortThreads / 32][kMaxRadix];   // 16 KB
+    extern __shared__ uint4 sort_smem_raw[];
+    SortScatterSmem& sm = *reinterpret_cast<SortScatterSmem*>(sort_smem_raw);
     const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (uint32_t w = 0; w < kSortThreads / 32; ++w)
-        for (uint32_t d = threadIdx.x; d < radix; d += kSortThreads) warp_hist[w][d] = 0;
-    __syncthreads();
+    for (uint32_t d = threadIdx.x; d < radix; d += kSortThreads)
+#pragma unroll
+        for (int w = 0; w < kSortWarps; ++w) sm.warp_hist[w][d] = 0;
     const SortTile t = tiles[blockIdx.x];
+    uint32_t* keys_s = sort_stage(keys_in + t.first, t.count, sm.keys);
+    unsigned long long* cards_s = sort_stage(vals_in + t.first, t.count, sm.cards);
+    __syncthreads();
 
     // each warp owns a contiguous run of kSortStrips * 32 keys (keeps the order stable)
     const uint32_t wlocal = warp * (kSortStrips * 32);
@@ -330,45 +392,75 @@ __global__ void __launch_bounds__(kSortThreads, 4) sort_scatter(const uint32_t* 
     {
         const uint32_t local = wlocal + (uint32_t)i * 32 + lane;
         const bool in = local < t.count;
-        key[i] = in ? keys_in[t.first + local] : 0xFFFFFFFFu;
+        key[i] = in ? keys_s[local] : 0xFFFFFFFFu;
         const uint32_t d = in ? ((key[i] >> shift) & mask) : 0xFFFFFFFFu;
         const unsigned peers = __match_any_sync(0xFFFFFFFFu, d);
-        const uint32_t before = in ? warp_hist[warp][d] : 0;
+        const uint32_t before = in ? sm.warp_hist[warp][d] : 0;
         rank[i] = before + __popc(peers & ((1u << lane) - 1));
         __syncwarp();
-        if (in && (__ffs(peers) - 1) == (int)lane) warp_hist[warp][d] = before + __popc(peers);
+        if (in && (__ffs(peers) - 1) == (int)lane) sm.warp_hist[warp][d] = before + __popc(peers);
         __syncwarp();
     }
     __syncthreads();
-    // per digit: turn per-warp counts into global bases
-    for (uint32_t d = threadIdx.x; d < radix; d += kSortThreads)
-    {
-        uint32_t run = offsets[sort_count_index(t, radix, d)];
+    // per digit (two per thread, radix <= 2 * kSortThreads): tile-local start of its run, global base, per-warp slots
+    uint32_t c2[2] = {0, 0};
 #pragma unroll
-        for (int w = 0; w < kSortThreads / 32; ++w)
+    for (int e = 0; e < 2; ++e)
+    {
+        const uint32_t d = 2u * threadIdx.x + (uint32_t)e;
+        if (d < radix)
+#pragma unroll
+            for (int w = 0; w < kSortWarps; ++w) c2[e] += sm.warp_hist[w][d];
+    }
+    uint32_t total;
+    uint32_t run = block_exclusive_scan<uint32_t, kSortThreads>(c2[0] + c2[1], total, sm.scan);
+#pragma unroll
+    for (int e = 0; e < 2; ++e)
+    {
+        const uint32_t d = 2u * threadIdx.x + (uint32_t)e;
+        if (d < radix)
         {
-            const uint32_t c = warp_hist[w][d];
-            warp_hist[w][d] = run;
-            run += c;
+            sm.gbase[d] = offsets[sort_count_index(t, radix, d)] - run;
+#pragma unroll
+            for (int w = 0; w < kSortWarps; ++w)
+            {
+                const uint32_t c = sm.warp_hist[w][d];
+                sm.warp_hist[w][d] = run;
+                run += c;
+            }
         }
     }
     __syncthreads();
+    // reorder: the keys (read into registers above), then the cards (read before the barrier, written after it)
+    unsigned long long card[kSortStrips];
 #pragma unroll
     for (int i = 0; i < kSortStrips; ++i)
     {
         const uint32_t local = wlocal + (uint32_t)i * 32 + lane;
         if (local < t.count)
         {
-            const uint32_t d = (key[i] >> shift) & mask;
-            const uint32_t dst = warp_hist[warp][d] + rank[i];
-            keys_out[dst] = key[i];
-            vals_out[dst] = vals_in[t.first + local];
-            if (next_counts)
-            {   // the chunk's keys stay inside the chunk: destination - first key of the chunk = place inside the chunk
-                const uint32_t chunk_first = t.first - t.blk * (uint32_t)kSortTile;
-                const uint32_t nt = (dst - chunk_first) / (uint32_t)kSortTile;
-                atomicAdd(&next_counts[(uint64_t)next_radix * t.cblk + (uint64_t)((key[i] >> next_shift) & next_mask) * t.nblk + nt], 1u);
-            }
+            rank[i] += sm.warp_hist[warp][(key[i] >> shift) & mask];
+            sm.keys[rank[i]] = key[i];
+        }
+        card[i] = local < t.count ? cards_s[local] : 0ull;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int i = 0; i < kSortStrips; ++i)
+        if (wlocal + (uint32_t)i * 32 + lane < t.count) sm.cards[rank[i]] = card[i];
+    __syncthreads();
+    // the chunk's keys stay inside the chunk: destination - first key of the chunk = place inside the chunk
+    const uint32_t chunk_first = t.first - t.blk * (uint32_t)kSortTile;
+    for (uint32_t s = threadIdx.x; s < t.count; s += kSortThreads)
+    {
+        const uint32_t k = sm.keys[s];
+        const uint32_t dst = sm.gbase[(k >> shift) & mask] + s;
+        keys_out[dst] = k;
+        vals_out[dst] = sm.cards[s];
+        if (next_counts)
+        {
+            const uint32_t nt = (dst - chunk_first) / (uint32_t)kSortTile;
+            atomicAdd(&next_counts[(uint64_t)next_radix * t.cblk + (uint64_t)((k >> next_shift) & next_mask) * t.nblk + nt], 1u);
         }
     }
 }
