@@ -530,23 +530,7 @@ int stage_finalize(fsb_ctx* c, Batch& b, cudaStream_t st)
     {
         sb.tile_off = b.tiles_host.size();
         sb.ctile_off = b.ctiles_host.size();
-        uint32_t cblk = 0;
-        for (uint32_t ci = sb.c0; ci < sb.c1; ++ci)
-        {
-            b.ctiles_host.push_back(cblk);
-            const uint64_t first = b.chunk_first_rec[ci] - sb.r0, cnt = b.chunk_first_rec[ci + 1] - b.chunk_first_rec[ci];
-            const uint32_t nblk = (uint32_t)((cnt + kSortTile - 1) / kSortTile);
-            for (uint32_t k = 0; k < nblk; ++k)
-            {
-                SortTile t{};
-                t.first = (uint32_t)(first + (uint64_t)k * kSortTile);
-                t.count = (uint32_t)std::min<uint64_t>(kSortTile, cnt - (uint64_t)k * kSortTile);
-                t.cblk = cblk; t.blk = k; t.nblk = nblk;
-                b.tiles_host.push_back(t);
-            }
-            cblk += nblk;
-        }
-        b.ctiles_host.push_back(cblk);
+        sort_tiles_build(b.chunk_first_rec.data() + sb.c0, sb.c1 - sb.c0, b.tiles_host, b.ctiles_host);
         sb.n_tiles = b.tiles_host.size() - sb.tile_off;
     }
     CUDA_TRY(c, b.d_chunk_tiles.ensure((b.ctiles_host.size() + 1) * 4));
@@ -936,7 +920,7 @@ int run_sub(fsb_ctx* c, Batch& b, const Sub& sb, fsb_ctx::Lane& L, cudaEvent_t* 
 
     // digit plan of the sort; K1 counts the first pass's digits while it writes the keys (scan_sort.cuh, ingest.cuh: SortSeed)
     int width[8];
-    const int passes = sort_plan((int)c->dp.key_bits, width);
+    sort_plan((int)c->dp.key_bits, width);
     const bool seeded = c->fused_hist && n && sub_chunks <= 32u;
     SortSeed seed{nullptr, nullptr, 0, 0, (uint32_t)kSortTile};
     if (seeded)
@@ -976,33 +960,11 @@ int run_sub(fsb_ctx* c, Batch& b, const Sub& sb, fsb_ctx::Lane& L, cudaEvent_t* 
     int cur = 0;
     if (n)
     {
-        const SortTile* tiles = b.d_sort_tiles.as<SortTile>() + sb.tile_off;
-        const uint32_t nblocks = (uint32_t)sb.n_tiles;
-        int shift = 0;
-        bool counted = seeded;                                       // the pass's digit counts are in d_counts already
-        for (int pass = 0; pass < passes; ++pass)
-        {
-            const uint32_t radix = 1u << width[pass], mask = radix - 1u;
-            const uint64_t ncounts = (uint64_t)radix * nblocks;
-            if (!counted)
-            {
-                sort_histogram<<<nblocks, kSortThreads, 0, st>>>(L.d_keys[cur].as<uint32_t>(), tiles, shift, mask, radix, L.d_counts.as<uint32_t>());
-                launches++;
-            }
-            launches += exclusive_scan<uint32_t, uint32_t>(L.d_counts.as<uint32_t>(), ncounts, L.d_counts_scan.as<uint32_t>(), L.d_scan_tmp.as<uint32_t>(), st);
-            // the scatter counts the digits of the next pass: a key's destination is the tile it will be read from
-            const bool count_next = c->fused_hist && pass + 1 < passes;
-            const uint32_t next_radix = count_next ? (1u << width[pass + 1]) : 0u;
-            if (count_next) CUDA_TRY(c, cudaMemsetAsync(L.d_counts.p, 0, (size_t)next_radix * nblocks * 4, st));
-            CUDA_TRY(c, cudaFuncSetAttribute(sort_scatter, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SortScatterSmem)));
-            sort_scatter<<<nblocks, kSortThreads, sizeof(SortScatterSmem), st>>>(L.d_keys[cur].as<uint32_t>(), L.d_cards[cur].as<unsigned long long>(), tiles, shift, mask, radix,
-                                                            L.d_counts_scan.as<uint32_t>(), L.d_keys[cur ^ 1].as<uint32_t>(), L.d_cards[cur ^ 1].as<unsigned long long>(),
-                                                            count_next ? L.d_counts.as<uint32_t>() : nullptr, shift + width[pass], next_radix ? next_radix - 1u : 0u, next_radix);
-            counted = count_next;
-            shift += width[pass];
-            launches++;
-            cur ^= 1;
-        }
+        uint32_t* const keys[2] = {L.d_keys[0].as<uint32_t>(), L.d_keys[1].as<uint32_t>()};
+        unsigned long long* const cards[2] = {L.d_cards[0].as<unsigned long long>(), L.d_cards[1].as<unsigned long long>()};
+        // seeded: the first pass's digit counts are in d_counts already
+        CUDA_TRY(c, sort_passes(keys, cards, b.d_sort_tiles.as<SortTile>() + sb.tile_off, (uint32_t)sb.n_tiles, (int)c->dp.key_bits, seeded, c->fused_hist,
+                                L.d_counts.as<uint32_t>(), L.d_counts_scan.as<uint32_t>(), L.d_scan_tmp.as<uint32_t>(), st, cur, launches));
     }
     const uint32_t* sorted_keys = L.d_keys[cur].as<uint32_t>();
     const unsigned long long* sorted_cards = L.d_cards[cur].as<unsigned long long>();
@@ -1024,17 +986,8 @@ int run_sub(fsb_ctx* c, Batch& b, const Sub& sb, fsb_ctx::Lane& L, cudaEvent_t* 
                  L.d_flags.as<uint32_t>(), L.d_tbase.as<unsigned long long>()};
     if (fused)
     {
-        const unsigned nlay = (unsigned)((n + kLayBlock - 1) / kLayBlock);
-        LayState* states = L.d_lay_states.as<LayState>();
-        ChunkStart* cstart = L.d_chunk_start.as<ChunkStart>();
-        CUDA_TRY(c, cudaFuncSetAttribute(lay_reduce_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLayReduceSmem));
-        CUDA_TRY(c, cudaFuncSetAttribute(lay_apply_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLayApplySmem));
-        lay_reduce_kernel<<<nlay, kLayThreads, kLayReduceSmem, st>>>(n, P, S, b.min_len, states);
-        const unsigned ngroups = (nlay + kLayScanThreads - 1) / kLayScanThreads;
-        lay_scan_groups_kernel<<<ngroups, kLayScanThreads, 0, st>>>(states, nlay, states + nlay + 1);
-        lay_scan_finish_kernel<<<ngroups, kLayScanThreads, 0, st>>>(states, nlay, states + nlay + 1);
-        lay_apply_kernel<<<nlay, kLayThreads, kLayApplySmem, st>>>(n, sub_chunks, P, S, b.min_len, states, LayOut{pm, O, desc, cstart, L.d_nb.as<uint32_t>()});
-        chunk_summary_fused_kernel<<<sub_chunks, 128, 0, st>>>(B, cstart, desc, b.d_summary.as<ChunkSummary>() + sb.c0);
+        CUDA_TRY(c, lay_fused_launch(n, P, S, b.min_len, B, L.d_lay_states.as<LayState>(), LayOut{pm, O, desc, L.d_chunk_start.as<ChunkStart>(), L.d_nb.as<uint32_t>()},
+                                     b.d_summary.as<ChunkSummary>() + sb.c0, st));
         launches += 5;
     }
     else

@@ -138,10 +138,12 @@ __device__ __forceinline__ void lay_stage(const SortedView& S, uint64_t n, uint6
     }
     __syncwarp();
 }
-// the key in front of the thread's run (only the last run of a batch is partial, so the run in front is whole)
+// the key in front of the thread's run (only the last run of a batch is partial, so the run in front is whole); 0 for an empty
+// run, whose lane 0 would otherwise read behind the end of the keys
 __device__ __forceinline__ uint32_t lay_prev_key(const SortedView& S, const LayWarpIn& w, const LayRun& run)
 {
     const unsigned lane = threadIdx.x & 31;
+    if (!run.cnt) return 0u;
     return lane ? w.keys[lane - 1][kLayPerThread - 1] : (run.i0 ? S.skeys[run.i0 - 1] : 0u);
 }
 // the state of a thread's run, walked from its row
@@ -376,6 +378,29 @@ __global__ void __launch_bounds__(128) chunk_summary_fused_kernel(BatchView Bv, 
         s.raw_dna = raw[0]; s.raw_head = raw[1];
         out[c] = s;
     }
+}
+
+// block states and group totals the layout of n records takes in `states`
+inline uint64_t lay_states_count(uint64_t n)
+{
+    const uint64_t nlay = (n + kLayBlock - 1) / kLayBlock;
+    return nlay + 1 + (nlay + kLayScanThreads - 1) / kLayScanThreads;
+}
+
+// The five launches of the layout of n >= 1 sorted records whose reads all have `uniform_len` bases, in B.n_chunks chunks.
+inline cudaError_t lay_fused_launch(uint64_t n, const DeviceParams& P, const SortedView& S, uint32_t uniform_len, const BatchView& B, LayState* states,
+                                    const LayOut& out, ChunkSummary* summary, cudaStream_t st)
+{
+    const unsigned nlay = (unsigned)((n + kLayBlock - 1) / kLayBlock);
+    if (cudaError_t e = cudaFuncSetAttribute(lay_reduce_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLayReduceSmem)) return e;
+    if (cudaError_t e = cudaFuncSetAttribute(lay_apply_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLayApplySmem)) return e;
+    lay_reduce_kernel<<<nlay, kLayThreads, kLayReduceSmem, st>>>(n, P, S, uniform_len, states);
+    const unsigned ngroups = (nlay + kLayScanThreads - 1) / kLayScanThreads;
+    lay_scan_groups_kernel<<<ngroups, kLayScanThreads, 0, st>>>(states, nlay, states + nlay + 1);
+    lay_scan_finish_kernel<<<ngroups, kLayScanThreads, 0, st>>>(states, nlay, states + nlay + 1);
+    lay_apply_kernel<<<nlay, kLayThreads, kLayApplySmem, st>>>(n, B.n_chunks, P, S, uniform_len, states, out);
+    chunk_summary_fused_kernel<<<B.n_chunks, 128, 0, st>>>(B, out.chunk_start, out.desc, summary);
+    return cudaSuccess;
 }
 
 } // namespace fsb

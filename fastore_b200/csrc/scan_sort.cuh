@@ -8,7 +8,9 @@
 // keeps equal keys in input order.
 #pragma once
 
+#include <algorithm>
 #include <cstdint>
+#include <vector>
 #include <cuda_runtime.h>
 
 namespace fsb {
@@ -472,6 +474,67 @@ inline int sort_plan(int bits, int (&width)[8])
     const int base = bits / passes, rem = bits % passes;
     for (int p = 0; p < passes; ++p) width[p] = base + (p >= passes - rem ? 1 : 0);
     return passes;
+}
+
+// The sort tiles of one sub-batch of `n_chunks` chunks, chunk ci holding records [first_rec[ci], first_rec[ci + 1]): tiles of at
+// most kSortTile keys, every one inside its chunk, appended to `tiles`; per chunk the tiles of all earlier chunks, then their
+// total, appended to `ctiles`.
+inline void sort_tiles_build(const uint64_t* first_rec, uint32_t n_chunks, std::vector<SortTile>& tiles, std::vector<uint32_t>& ctiles)
+{
+    uint32_t cblk = 0;
+    for (uint32_t ci = 0; ci < n_chunks; ++ci)
+    {
+        ctiles.push_back(cblk);
+        const uint64_t first = first_rec[ci] - first_rec[0], cnt = first_rec[ci + 1] - first_rec[ci];
+        const uint32_t nblk = (uint32_t)((cnt + kSortTile - 1) / kSortTile);
+        for (uint32_t k = 0; k < nblk; ++k)
+        {
+            SortTile t{};
+            t.first = (uint32_t)(first + (uint64_t)k * kSortTile);
+            t.count = (uint32_t)std::min<uint64_t>(kSortTile, cnt - (uint64_t)k * kSortTile);
+            t.cblk = cblk; t.blk = k; t.nblk = nblk;
+            tiles.push_back(t);
+        }
+        cblk += nblk;
+    }
+    ctiles.push_back(cblk);
+}
+
+// The passes of the sort of one sub-batch over its `ntiles` sort tiles: keys[cur] / cards[cur] in, the other buffer of each
+// pair out, `cur` flipped once per pass.  counts takes (largest radix) * ntiles entries, counts_scan one more, scan_tmp
+// scan_num_tiles(counts) + 1.  `counted`: counts already holds the first pass's digit counts.  `fused_hist`: the scatter
+// counts the digits of the next pass (FSB_OPT_FUSED_HIST), which then needs no histogram launch.
+inline cudaError_t sort_passes(uint32_t* const keys[2], unsigned long long* const cards[2], const SortTile* tiles, uint32_t ntiles, int key_bits,
+                               bool counted, bool fused_hist, uint32_t* counts, uint32_t* counts_scan, uint32_t* scan_tmp, cudaStream_t st,
+                               int& cur, uint64_t& launches)
+{
+    int width[8];
+    const int passes = sort_plan(key_bits, width);
+    int shift = 0;
+    for (int pass = 0; pass < passes; ++pass)
+    {
+        const uint32_t radix = 1u << width[pass], mask = radix - 1u;
+        const uint64_t ncounts = (uint64_t)radix * ntiles;
+        if (!counted)
+        {
+            sort_histogram<<<ntiles, kSortThreads, 0, st>>>(keys[cur], tiles, shift, mask, radix, counts);
+            launches++;
+        }
+        launches += exclusive_scan<uint32_t, uint32_t>(counts, ncounts, counts_scan, scan_tmp, st);
+        // the scatter counts the digits of the next pass: a key's destination is the tile it will be read from
+        const bool count_next = fused_hist && pass + 1 < passes;
+        const uint32_t next_radix = count_next ? (1u << width[pass + 1]) : 0u;
+        if (count_next)
+            if (cudaError_t e = cudaMemsetAsync(counts, 0, (size_t)next_radix * ntiles * 4, st)) return e;
+        if (cudaError_t e = cudaFuncSetAttribute(sort_scatter, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SortScatterSmem))) return e;
+        sort_scatter<<<ntiles, kSortThreads, sizeof(SortScatterSmem), st>>>(keys[cur], cards[cur], tiles, shift, mask, radix, counts_scan, keys[cur ^ 1], cards[cur ^ 1],
+                                                                             count_next ? counts : nullptr, shift + width[pass], next_radix ? next_radix - 1u : 0u, next_radix);
+        counted = count_next;
+        shift += width[pass];
+        launches++;
+        cur ^= 1;
+    }
+    return cudaSuccess;
 }
 
 } // namespace fsb

@@ -278,64 +278,109 @@ extern "C" int emul_pack(const fsb_params* p, const fsb_chunk* ch, uint8_t* meta
 // (positions, bin descriptors, bin count), or a negative value when the chunk's reads differ in length.
 #include "../../fastore_b200/csrc/layout_core.cuh"
 
-extern "C" long emul_layout_fused(const fsb_params* p, const fsb_chunk* ch, uint32_t per_thread, uint32_t threads)
+namespace {
+
+// A chunk's records sorted as the device sorts a batch: by chunk : signature, stably; records from `split` on form a second chunk.
+// Returns the reads' common length, 0 when they differ or there are none, or -2 when the signatures fail.
+long sorted_case(const fsb_params* p, const fsb_chunk* ch, uint64_t split, std::vector<uint32_t>& keys, std::vector<uint64_t>& cards)
 {
     const DeviceParams P = make_device_params(*p);
     const uint64_t n = ch->n_records;
+    keys.clear();
+    cards.clear();
     if (n == 0) return 0;
     std::vector<uint32_t> sig(n), info(n);
     if (emul_signatures(p, ch, sig.data(), info.data()) != FSB_OK) return -2;
     const bool pe = P.paired != 0;
     uint32_t ulen = ch->records[0][0].seq_len;
     for (int m = 0; m < (pe ? 2 : 1); ++m)
-        for (uint64_t i = 0; i < n; ++i) if (ch->records[m][i].seq_len != ulen) return -1;
-    // sorted keys and cards (one chunk: chunk bits 0; a second pseudo-chunk is made of the upper half to exercise chunk starts)
+        for (uint64_t i = 0; i < n; ++i) if (ch->records[m][i].seq_len != ulen) ulen = 0;
     std::vector<uint32_t> order(n);
     std::iota(order.begin(), order.end(), 0u);
-    const uint64_t half = n / 2;
-    auto chunk_of_rec = [&](uint32_t r) { return r < half ? 0u : 1u; };
-    std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) {
-        const uint64_t ka = ((uint64_t)chunk_of_rec(a) << P.key_bits) | sig[a], kb = ((uint64_t)chunk_of_rec(b) << P.key_bits) | sig[b];
-        return ka < kb; });
-    std::vector<uint32_t> keys(n);
-    std::vector<uint64_t> cards(n);
+    auto key_of = [&](uint32_t r) { return ((r < split ? 0u : 1u) << P.key_bits) | sig[r]; };
+    std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return key_of(a) < key_of(b); });
+    keys.resize(n);
+    cards.resize(n);
     for (uint64_t i = 0; i < n; ++i)
     {
         const uint32_t r = order[i];
-        keys[i] = (chunk_of_rec(r) << P.key_bits) | sig[r];
+        keys[i] = key_of(r);
         cards[i] = card_make(r, info[r], ch->records[0][r].seq_len, pe ? ch->records[1][r].seq_len : 0, P.has_headers ? ch->records[0][r].head_len : 0);
     }
-    // ---- the plain walk (the way run_pack above lays a chunk out) --------------------------------------------
-    std::vector<uint64_t> want_at[4];
+    return ulen;
+}
+
+// The plain walk over sorted records (the way run_pack above lays a chunk out): every record's first bit per stream, every bin's descriptor.
+void plain_walk(const DeviceParams& P, const uint32_t* keys, const uint64_t* cards, uint64_t n, uint32_t ulen, std::vector<uint64_t> (&want_at)[4],
+                std::vector<fsb_bin_descriptor>& want_desc)
+{
     for (auto& v : want_at) v.resize(n);
-    std::vector<fsb_bin_descriptor> want_desc;
+    uint64_t pos[4] = {0, 0, 0, 0}, start[4] = {0, 0, 0, 0};
+    fsb_bin_descriptor d{};
+    for (uint64_t i = 0; i < n; ++i)
     {
-        uint64_t pos[4] = {0, 0, 0, 0}, start[4] = {0, 0, 0, 0};
-        fsb_bin_descriptor d{};
-        for (uint64_t i = 0; i < n; ++i)
+        const bool st = i == 0 || keys[i] != keys[i - 1];
+        if (st)
         {
-            const bool st = i == 0 || keys[i] != keys[i - 1];
-            if (st)
-            {
-                for (int s = 0; s < 4; ++s) { pos[s] = (pos[s] + 7) & ~7ull; start[s] = pos[s]; }
-                pos[0] += 17;
-                d = fsb_bin_descriptor{};
-                d.signature = keys[i] & ((1u << P.key_bits) - 1u);
-            }
-            const uint64_t c = cards[i];
-            const bool nbin = d.signature == P.nbin;
-            const ReadBits rb = read_bit_lengths(P, nbin, card_info(c), card_lenA(c), card_lenB(c), card_head(c), ulen, ulen);
-            const uint32_t bits[4] = {rb.meta, rb.dna, rb.qua, rb.head};
-            for (int s = 0; s < 4; ++s) { want_at[s][i] = pos[s]; pos[s] += bits[s]; }
-            d.records_count++; d.raw_dna_size += card_lenA(c) + card_lenB(c); d.raw_head_size += P.has_headers ? card_head(c) : 0;
-            if (i + 1 == n || keys[i + 1] != keys[i])
-            {
-                d.meta_size = (((pos[0] + 7) & ~7ull) - start[0]) >> 3; d.dna_size = (((pos[1] + 7) & ~7ull) - start[1]) >> 3;
-                d.qua_size = (((pos[2] + 7) & ~7ull) - start[2]) >> 3; d.head_size = (((pos[3] + 7) & ~7ull) - start[3]) >> 3;
-                want_desc.push_back(d);
-            }
+            for (int s = 0; s < 4; ++s) { pos[s] = (pos[s] + 7) & ~7ull; start[s] = pos[s]; }
+            pos[0] += 17;
+            d = fsb_bin_descriptor{};
+            d.signature = keys[i] & ((1u << P.key_bits) - 1u);
+        }
+        const uint64_t c = cards[i];
+        const bool nbin = d.signature == P.nbin;
+        const ReadBits rb = read_bit_lengths(P, nbin, card_info(c), card_lenA(c), card_lenB(c), card_head(c), ulen, ulen);
+        const uint32_t bits[4] = {rb.meta, rb.dna, rb.qua, rb.head};
+        for (int s = 0; s < 4; ++s) { want_at[s][i] = pos[s]; pos[s] += bits[s]; }
+        d.records_count++; d.raw_dna_size += card_lenA(c) + card_lenB(c); d.raw_head_size += P.has_headers ? card_head(c) : 0;
+        if (i + 1 == n || keys[i + 1] != keys[i])
+        {
+            d.meta_size = (((pos[0] + 7) & ~7ull) - start[0]) >> 3; d.dna_size = (((pos[1] + 7) & ~7ull) - start[1]) >> 3;
+            d.qua_size = (((pos[2] + 7) & ~7ull) - start[2]) >> 3; d.head_size = (((pos[3] + 7) & ~7ull) - start[3]) >> 3;
+            want_desc.push_back(d);
         }
     }
+}
+
+} // namespace
+
+// sorted_case for the tests: keys / cards must hold ch->n_records entries
+extern "C" long emul_sorted_case(const fsb_params* p, const fsb_chunk* ch, uint64_t split, uint32_t* keys_out, uint64_t* cards_out)
+{
+    std::vector<uint32_t> keys;
+    std::vector<uint64_t> cards;
+    const long ulen = sorted_case(p, ch, split, keys, cards);
+    std::copy(keys.begin(), keys.end(), keys_out);
+    std::copy(cards.begin(), cards.end(), cards_out);
+    return ulen;
+}
+
+// plain_walk for the tests: at[4 * n]; desc must have room for every bin; returns the number of bins
+extern "C" uint64_t emul_plain_walk(const fsb_params* p, const uint32_t* keys, const uint64_t* cards, uint64_t n, uint32_t ulen, uint64_t* at, fsb_bin_descriptor* desc)
+{
+    std::vector<uint64_t> want_at[4];
+    std::vector<fsb_bin_descriptor> want_desc;
+    plain_walk(make_device_params(*p), keys, cards, n, ulen, want_at, want_desc);
+    for (int s = 0; s < 4; ++s) std::copy(want_at[s].begin(), want_at[s].end(), at + s * n);
+    std::copy(want_desc.begin(), want_desc.end(), desc);
+    return want_desc.size();
+}
+
+extern "C" long emul_layout_fused(const fsb_params* p, const fsb_chunk* ch, uint32_t per_thread, uint32_t threads)
+{
+    const DeviceParams P = make_device_params(*p);
+    const uint64_t n = ch->n_records;
+    if (n == 0) return 0;
+    // sorted keys and cards (one chunk: chunk bits 0; a second pseudo-chunk is made of the upper half to exercise chunk starts)
+    std::vector<uint32_t> keys;
+    std::vector<uint64_t> cards;
+    const long sc = sorted_case(p, ch, n / 2, keys, cards);
+    if (sc < 0) return sc;
+    if (sc == 0) return -1;
+    const uint32_t ulen = (uint32_t)sc;
+    std::vector<uint64_t> want_at[4];
+    std::vector<fsb_bin_descriptor> want_desc;
+    plain_walk(P, keys.data(), cards.data(), n, ulen, want_at, want_desc);
     // ---- the three phases ------------------------------------------------------------------------------------------
     const uint64_t per_block = (uint64_t)per_thread * threads;
     const uint64_t nblocks = (n + per_block - 1) / per_block;
@@ -393,6 +438,85 @@ extern "C" long emul_layout_fused(const fsb_params* p, const fsb_chunk* ch, uint
     if (block_state[nblocks].nstarts != want_desc.size()) bad++;
     for (size_t b = 0; b < want_desc.size(); ++b) if (std::memcmp(&got_desc[b], &want_desc[b], sizeof(fsb_bin_descriptor)) != 0) bad++;
     return bad;
+}
+
+// What lay_apply (layout_fused.cuh) must hand K4 for n sorted records whose reads all have `ulen` bases, in n_chunks chunks, as a
+// plain walk record after record: no LayState, no scan.  Outputs as tests/gpu_harness/sort_layout.cu's h_layout returns them:
+//   loc[k][i]    record i's first bit in stream k minus b0 plus (b0 & 127), b0 = the first bit of its 32-record tile: the tile's first
+//                record, or the first byte of the bin that record opens (0 for the title stream when titles are dropped)
+//   binfo[i]     ulen | ulen << 8 | opens its bin << 16 | N-bin << 17
+//   tbase        [tile][k] = b0, and [tiles][k] = the end of stream k rounded up to a byte
+//   desc, nb     the bins; chunk_start[5 * c] = the first bin and the first byte of every stream of chunk c (chunks that hold records
+//                only), then the same for the end of the batch
+//   cleared      the stream words K4 shares between two tiles, which the layout zeroes, as k << 60 | word; returns their number
+extern "C" uint64_t emul_layout_tables(const fsb_params* p, const uint32_t* keys, const uint64_t* cards, uint64_t n, uint32_t ulen, uint32_t n_chunks,
+                                       uint32_t* loc, uint32_t* binfo, uint64_t* tbase, fsb_bin_descriptor* desc, uint64_t* chunk_start, uint32_t* nb,
+                                       uint64_t* cleared)
+{
+    const DeviceParams P = make_device_params(*p);
+    const uint32_t key_mask = (1u << P.key_bits) - 1u;
+    uint64_t pos[4] = {0, 0, 0, 0}, start[4] = {0, 0, 0, 0}, b0[4] = {0, 0, 0, 0};
+    uint64_t n_cleared = 0;
+    auto clear = [&](int k, uint64_t bit) { if (bit & 31u) cleared[n_cleared++] = ((uint64_t)k << 60) | (bit >> 5); };
+    uint32_t bins = 0;
+    fsb_bin_descriptor d{};
+    for (uint64_t i = 0; i < n; ++i)
+    {
+        const uint32_t key = keys[i];
+        const bool opens = i == 0 || key != keys[i - 1];
+        const bool nbin = (key & key_mask) == P.nbin;
+        if (opens)
+        {
+            for (int k = 0; k < 4; ++k) { pos[k] = roundup8(pos[k]); start[k] = pos[k]; }
+            pos[0] += 17;                                              // minLen, maxLen, hasReadGroups
+            bins++;
+            d = fsb_bin_descriptor{};
+            d.signature = key & key_mask;
+            if (i == 0 || (key >> P.key_bits) != (keys[i - 1] >> P.key_bits))
+            {
+                uint64_t* cs = chunk_start + 5 * (key >> P.key_bits);
+                cs[0] = bins - 1;
+                for (int k = 0; k < 4; ++k) cs[1 + k] = start[k] >> 3;
+            }
+        }
+        const uint64_t c = cards[i];
+        const ReadBits rb = read_bit_lengths(P, nbin, card_info(c), card_lenA(c), card_lenB(c), card_head(c), ulen, ulen);
+        const uint32_t bits[4] = {rb.meta, rb.dna, rb.qua, rb.head};
+        for (int k = 0; k < 4; ++k)
+        {
+            const bool has = k < 3 || P.has_headers;
+            if (i % 32 == 0)
+            {
+                b0[k] = has ? (opens ? start[k] : pos[k]) : 0;
+                tbase[4 * (i / 32) + k] = b0[k];
+                clear(k, b0[k]);
+            }
+            loc[k * n + i] = has ? (uint32_t)(pos[k] - b0[k] + (b0[k] & 127u)) : 0u;
+            pos[k] += bits[k];
+        }
+        binfo[i] = (ulen & 0xFFu) | ((ulen & 0xFFu) << 8) | (opens ? 0x10000u : 0u) | (nbin ? 0x20000u : 0u);
+        d.records_count++;
+        d.raw_dna_size += card_lenA(c) + card_lenB(c);
+        d.raw_head_size += P.has_headers ? card_head(c) : 0u;
+        if (i + 1 == n || keys[i + 1] != key)
+        {
+            d.meta_size = (roundup8(pos[0]) - start[0]) >> 3; d.dna_size = (roundup8(pos[1]) - start[1]) >> 3;
+            d.qua_size = (roundup8(pos[2]) - start[2]) >> 3; d.head_size = (roundup8(pos[3]) - start[3]) >> 3;
+            desc[bins - 1] = d;
+        }
+    }
+    const uint64_t tiles = (n + 31) / 32;
+    uint64_t* cs = chunk_start + 5 * (uint64_t)n_chunks;
+    cs[0] = bins;
+    for (int k = 0; k < 4; ++k)
+    {
+        const bool has = k < 3 || P.has_headers;
+        tbase[4 * tiles + k] = has ? roundup8(pos[k]) : 0;
+        clear(k, tbase[4 * tiles + k]);
+        cs[1 + k] = roundup8(pos[k]) >> 3;
+    }
+    *nb = bins;
+    return n_cleared;
 }
 
 // ================================================================================================
